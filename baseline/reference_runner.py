@@ -1,4 +1,4 @@
-"""Drive the UNMODIFIED reference (baseline/_ref/, installed by baseline/install_reference.py) through its own public API:
+"""Drive the UNMODIFIED reference (oracle/_ref/, installed by oracle/install_reference.py) through its own public API:
 `Tacotron()` + `TacotronLoss` from modules/tacotron2.py, configured by its own params/*.json -- no code of this repository on that path.
 
 Used by `bench.py --impl reference` (CPU, all host threads it can use) and by bench.py's extra baselines (the mandated cfg-1 CPU
@@ -10,7 +10,7 @@ import sys
 import time
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.path.join(HERE, '_ref')
+REF = os.path.join(os.path.dirname(HERE), 'oracle', '_ref')
 
 
 def available():
@@ -25,7 +25,7 @@ def load():
     global _loaded
     if _loaded is None:
         if not available():
-            raise RuntimeError('baseline/_ref is not installed: run `python baseline/install_reference.py` where /root/reference exists')
+            raise RuntimeError('oracle/_ref is not installed: run `python oracle/install_reference.py` where the original sources exist')
         sys.dont_write_bytecode = True
         if REF not in sys.path:
             sys.path.insert(0, REF)

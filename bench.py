@@ -3,7 +3,7 @@
 
     python bench.py --gpus 1 --steps 5 --warmup 3                    # this framework, 1 GPU
     torchrun --nproc-per-node N ... bench.py --gpus N ...             # data parallel, one rank per GPU, NCCL all-reduce
-    python bench.py --impl reference --steps 2 --warmup 1             # CPU reference arm (unmodified reference from baseline/_ref, host cores)
+    python bench.py --impl reference --steps 2 --warmup 1             # CPU reference arm (unmodified reference from oracle/_ref, host cores)
 
 A "step" is one training step of the named configuration on one synthetic batch per GPU: embedding -> encoder ->
 fused decoder -> postnet -> TacotronLoss -> backward (-> gradient all-reduce when N > 1).  Optimizer, data loading
@@ -45,7 +45,12 @@ def parse():
     ap.add_argument('--breakdown', default='', help='write a per-kernel device-time table of one extra (untimed) step to this file')
     ap.add_argument('--precision', default='bf16', choices=['bf16', 'fp32'],
                     help="bf16: tensor-core operands, fp32 master/state (BASELINE configs[1]); fp32: exact parity mode")
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='after the timed steps, write what the last timed step returned (the loss and every parameter gradient) as DIR/<name>.npy')
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    return a
 
 
 def workload(a):
@@ -148,6 +153,30 @@ def measured_peaks():
     return 6650.0, 'fallback (B200_PROFILING.md)'
 
 
+DUMP_SAMPLE = 1 << 16      # elements kept of a larger gradient: the 152 gradients of the largest configuration stay below 64 MB
+
+
+def dump_outputs(directory, model, loss):
+    """What a training step hands its caller: the loss and every parameter's gradient, written as DIR/loss.npy and DIR/grad.<parameter
+    name>.npy in float32.  A gradient of more than DUMP_SAMPLE elements is stored at DUMP_SAMPLE fixed positions of its flattened
+    values (seeded, so the same for every run and every build), which lets two builds be compared output for output."""
+    import numpy as np
+    import torch
+    arrays = {'loss': loss.detach().float().cpu().numpy()}
+    for name, p in model.named_parameters():
+        g = p.grad.detach()
+        if g.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(g.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            g = g.flatten()[idx.to(g.device)]
+        arrays['grad.' + name] = g.float().cpu().numpy()
+    total = sum(v.nbytes for v in arrays.values())
+    if total > 64 << 20:
+        raise SystemExit(f'--dump-outputs: {total} bytes exceed the 64 MB bound')
+    os.makedirs(directory, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(directory, name + '.npy'), v)
+
+
 class ClockSampler:
     """nvidia-smi clocks / throttle reasons DURING the timed region (profiling recipe's clocks line)."""
     Q = 'clocks.sm,clocks.max.sm,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown,' \
@@ -239,7 +268,7 @@ def config_dict(a, world, B, L, T):
 def reference_cpu(a, steps, warmup):
     """The reference's own CPU implementation of the path on the host cores, on a BOUNDED sample of the workload: the same batch
     size / text length, but only the first `--ref-frames` of the T frames per utterance (a full T = 900 step of B = 60 takes ~1 min).
-    baseline/_ref (the unmodified reference) when installed, else the oracle port."""
+    oracle/_ref (the unmodified reference) when installed, else the oracle port."""
     hp, B, L, T = workload(a)
     Ts = min(a.ref_frames, T)
     sys.path.insert(0, os.path.join(ROOT, 'baseline'))
@@ -256,12 +285,12 @@ def reference_cpu(a, steps, warmup):
             if per_frame > 0:
                 extra = {'second_sample_frames': Ts // 2, 'second_sample_s_per_step': r2['s_per_step'], 'fixed_s': fixed,
                          's_per_frame_step': per_frame, 'extrapolated_full_T_frames_per_s': B * T / (fixed + per_frame * T)}
-        sample = (f'UNMODIFIED reference (baseline/_ref: Tacotron.forward + TacotronLoss + backward, torch {_torch_version()} CPU fp32), '
+        sample = (f'UNMODIFIED reference (oracle/_ref: Tacotron.forward + TacotronLoss + backward, torch {_torch_version()} CPU fp32), '
                   f'{a.config} B={B} L={L}, first {Ts} of T={T} frames per utterance, {steps} timed step(s), threads scanned {r["thread_scan"]}')
         return {'value': r['frames_per_s'], 'unit': UNIT, 'cores': r['cores'], 'kind': 'reference', 'sample': sample,
                 'host_cores': os.cpu_count(), 'sample_frames': Ts, 'extrapolation': extra}, r['s_per_step']
     fps, med, cores, sample = cpu_oracle_frames_per_s(a, steps, warmup, sample_frames=min(Ts, 24))
-    return {'value': fps, 'unit': UNIT, 'cores': cores, 'kind': 'port', 'sample': sample + ' (baseline/_ref not installed)',
+    return {'value': fps, 'unit': UNIT, 'cores': cores, 'kind': 'port', 'sample': sample + ' (oracle/_ref not installed)',
             'host_cores': os.cpu_count(), 'sample_frames': min(Ts, 24)}, med
 
 
@@ -292,7 +321,7 @@ def extra_baselines(a, threads):
     sys.path.insert(0, os.path.join(ROOT, 'baseline'))
     import reference_runner as R
     if not R.available():
-        return {'unavailable': 'baseline/_ref not installed'}
+        return {'unavailable': 'oracle/_ref not installed'}
     out = {}
     hp, B, L, T = workload(a)
     try:
@@ -378,13 +407,14 @@ def run_b200(a):
         return loss
 
     def timed(n, from_host):
-        """n steps bracketed by barrier + synchronize; device time by CUDA events; returns (max-over-ranks ms, last loss)."""
+        """n steps bracketed by barrier + synchronize; device time by CUDA events; returns (max-over-ranks ms, last loss read on the host
+        (from_host only), last loss tensor)."""
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        loss_val = None
+        loss_val, loss = None, None
         for _ in range(n):
             if from_host and graphed is not None:
                 batch = host                       # GraphedTrainStep copies the pinned host tensors into its static device buffers
@@ -399,7 +429,7 @@ def run_b200(a):
         if world > 1:
             dist.barrier()
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms), loss_val
+        return float(ms), loss_val, loss
 
     # the clock sampler (an nvidia-smi child process) starts BEFORE the warm-up: its NVML initialisation briefly contends with
     # the CUDA driver, which must not land inside the timed region
@@ -416,9 +446,11 @@ def run_b200(a):
         _lib.kernel_timing(True)          # CUDA events on the launching stream around the dominant kernels, inside the timed steps
     if ncu_range:
         torch.cuda.profiler.start()
-    ms, _ = timed(a.steps, from_host=False)
+    ms, _, last_loss = timed(a.steps, from_host=False)
     if ncu_range:
         torch.cuda.profiler.stop()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, model, last_loss)   # before the steps below overwrite the gradients
     launches = (_lib.launch_count() - n0) if graphed is None else launches_per_step * a.steps
     if graphed is not None:
         # events cannot be timed inside a replayed graph: the per-kernel durations come from the SAME kernels issued eagerly, a.steps
@@ -433,7 +465,7 @@ def run_b200(a):
     _lib.kernel_timing(False)
     dec_ms = [s.elapsed_time(e) for s, e in F.PROFILE.get('decoder_fwd', [])]
     decb_ms = [s.elapsed_time(e) for s, e in F.PROFILE.get('decoder_bwd', [])]
-    ms_e2e, loss_val = timed(a.steps, from_host=True)
+    ms_e2e, loss_val, _ = timed(a.steps, from_host=True)
     clocks = sampler.stop() if rank == 0 else None
     if a.breakdown and rank == 0:       # CUPTI kernel times of ONE extra step (not part of any reported number)
         from torch.profiler import profile, ProfilerActivity

@@ -55,6 +55,48 @@ class Golden:
         return {k: (v if k == 'teacher' else v.to(dtype)) for k, v in self.tape.items()}
 
 
+SAMPLE_MAX = 8192
+
+
+def sample_index(numel):
+    """Fixed, seeded flat positions at which a tensor larger than SAMPLE_MAX elements is stored in a golden file (None: stored whole)."""
+    if numel <= SAMPLE_MAX:
+        return None
+    return torch.randperm(numel, generator=torch.Generator().manual_seed(0))[:SAMPLE_MAX].sort().values
+
+
+def golden_array(t):
+    """What a golden file stores of `t`: the tensor itself, or its values at sample_index(t.numel())."""
+    t = t.detach().cpu()
+    idx = sample_index(t.numel())
+    return t if idx is None else t.flatten()[idx]
+
+
+def digest(t):
+    """float64 [sum, sum of squares, position-weighted sum]: pins a regenerated tensor (weights, inputs) to the one a fixture was made from."""
+    v = t.detach().cpu().double().flatten()
+    return torch.stack([v.sum(), (v * v).sum(), (v * torch.linspace(-1.0, 1.0, v.numel(), dtype=torch.float64)).sum()])
+
+
+class ModuleGolden:
+    """One case of tests/golden/modules_*.npz (tests/golden/make_golden_modules.py): arrays by name, as float64 torch tensors."""
+
+    def __init__(self, file, case):
+        z = np.load(os.path.join(GOLDEN_DIR, file + '.npz'))
+        self.a = {k[len(case) + 1:]: torch.from_numpy(z[k]).double() for k in z.files if k.startswith(case + '.')}
+
+    def __getitem__(self, name):
+        return self.a[name]
+
+    def check_digest(self, name, t):
+        got, want = digest(t), self.a['digest.' + name]
+        assert torch.allclose(got, want, rtol=1e-9, atol=1e-9), f'{name}: regenerated {got.tolist()} != fixture {want.tolist()}'
+
+    def assert_close(self, actual, name, rtol, atol):
+        """`actual` (whole tensor) against the stored (possibly sampled) reference values of `name`."""
+        assert_close(golden_array(actual), self.a[name], rtol, atol, name)
+
+
 def max_abs(a, b):
     return float((a.double() - b.double()).abs().max()) if a.numel() else 0.0
 

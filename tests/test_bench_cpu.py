@@ -1,4 +1,4 @@
-"""CPU checks of bench.py: the reference arm (the unmodified reference from baseline/_ref when installed, else the oracle port, on the
+"""CPU checks of bench.py: the reference arm (the unmodified reference from oracle/_ref when installed, else the oracle port, on the
 host cores) prints one well-formed JSON line, and the roofline bookkeeping reproduces the SURVEY section 8d figures."""
 import json
 import os
@@ -23,6 +23,30 @@ def test_bytes_fwd_step_matches_survey_table():
     assert abs(both / 1e6 - 42.6) < 0.05 and abs(e['frac'] - 0.283) < 0.002 and abs(e['frac_fp32_naive'] - 0.5655) < 0.002
 
 
+def test_dump_outputs_writes_loss_and_gradients(tmp_path):
+    """--dump-outputs: the loss and one float32 array per parameter gradient; a gradient above DUMP_SAMPLE elements is kept at the
+    same seeded positions on every call."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    torch.manual_seed(0)
+    model = torch.nn.Sequential(torch.nn.Linear(300, 300), torch.nn.Linear(300, 2))
+    loss = model(torch.randn(4, 300)).square().mean()
+    loss.backward()
+    for d in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / d), model, loss)
+    names = sorted(p.name for p in (tmp_path / 'a').iterdir())
+    assert names == ['grad.0.bias.npy', 'grad.0.weight.npy', 'grad.1.bias.npy', 'grad.1.weight.npy', 'loss.npy']
+    for n in names:
+        a, b = np.load(tmp_path / 'a' / n), np.load(tmp_path / 'b' / n)
+        assert a.dtype == np.float32 and np.array_equal(a, b), n
+    assert float(np.load(tmp_path / 'a' / 'loss.npy')) == float(loss.detach())
+    assert np.array_equal(np.load(tmp_path / 'a' / 'grad.1.weight.npy'), model[1].weight.grad.numpy())
+    big = np.load(tmp_path / 'a' / 'grad.0.weight.npy')
+    assert big.shape == (bench.DUMP_SAMPLE,) and set(big.tolist()) <= set(model[0].weight.grad.flatten().tolist())
+
+
 def test_reference_arm_prints_contract_line():
     env = dict(os.environ, OMP_NUM_THREADS='4')
     res = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--impl', 'reference', '--steps', '1', '--warmup', '0',
@@ -32,7 +56,7 @@ def test_reference_arm_prints_contract_line():
     for key in ('impl', 'metric', 'value', 'unit', 'n_gpus', 'steps', 'warmup', 'ms_per_step', 'higher_is_better', 'scaling', 'dtype', 'data',
                 'config', 'cpu_baseline', 'e2e'):
         assert key in line, key
-    installed = os.path.exists(os.path.join(ROOT, 'baseline', '_ref', 'modules', 'tacotron2.py'))
+    installed = os.path.exists(os.path.join(ROOT, 'oracle', '_ref', 'modules', 'tacotron2.py'))
     assert line['impl'] == 'reference' and line['value'] > 0 and line['cpu_baseline']['kind'] == ('reference' if installed else 'port')
     # the bounded sample is named: the arm never claims the full T
     assert line['config']['reference_sample_frames'] == 12 and 'first 12 of the T=900' in line['config']['workload']

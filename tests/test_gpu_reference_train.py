@@ -1,5 +1,5 @@
 """"train.py calls into it unchanged" (north_star, SURVEY 8b): the reference's OWN `train()` function body
-(baseline/_ref/train.py:29-95, byte-identical copy of /root/reference/train.py) drives THIS package for two optimisation steps.
+(oracle/_ref/train.py:29-95, a byte-identical copy of the original project's train.py installed by build()) drives THIS package for two optimisation steps.
 
 train.py is imported as it is; only what it imports at module level is substituted:
   params.params, modules.tacotron2, utils (lengths_to_mask, to_gpu)  -> this package (the two import lines INTEGRATION.md names)
@@ -18,7 +18,7 @@ import torch
 from helpers import ROOT
 
 pytestmark = pytest.mark.gpu
-TRAIN_PY = os.path.join(ROOT, 'baseline', '_ref', 'train.py')
+TRAIN_PY = os.path.join(ROOT, 'oracle', '_ref', 'train.py')
 
 
 @pytest.fixture(scope='module', autouse=True)
@@ -70,7 +70,7 @@ def _import_reference_train(logged):
     return mod
 
 
-@pytest.mark.skipif(not os.path.exists(TRAIN_PY), reason='baseline/_ref (the unmodified reference) is not installed')
+@pytest.mark.skipif(not os.path.exists(TRAIN_PY), reason='oracle/_ref (the unmodified reference) is not installed')
 @pytest.mark.parametrize('config', ['generated_switching', 'ljspeech'])
 def test_reference_train_function_runs_on_this_package(config):
     from multilingual_text_to_speech_b200 import configs
