@@ -15,6 +15,7 @@
 // the product.  Saved tensors (activated gates, hs, cs) keep the layout of the per-step chain, which remains the fallback for
 // shapes this kernel does not take (H % 32 != 0 or H > 256).
 #include "decoder_internal.cuh"
+#include "ptx.cuh"
 
 namespace b200tts {
 
@@ -36,20 +37,7 @@ struct BiLoopArgs {
     const int* lengths;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ uint32_t peer_addr(const void* local_smem, uint32_t rank) {
-    uint32_t ra;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(local_smem)), "r"(rank));
-    return ra;
-}
-__device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) { asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory"); }
-__device__ __forceinline__ void st_cluster_f32x4(uint32_t addr, float4 v) {
-    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
+using namespace tcx;
 
 // ------------------------------------------------------------------------------------------------
 // forward: z[b, row] = sum_k h_prev[b, k] W_hh[row, k]; thread = (gate row, 4 utterances) for the product, (utterance, unit) for the cell
@@ -84,7 +72,7 @@ __global__ void __launch_bounds__(RT, 1) bilstm_fwd_loop_kernel(const BiLoopArgs
     const int prow = tid & (RROWS - 1), pb0 = (tid >> 7) * 4;
     const size_t dirBH = (size_t)dir * (L + 1) * B * H, dirG = (size_t)dir * L * B * 4 * H;
     if (cvalid_b) { p.hs[dirBH + (size_t)bglob * H + u] = 0.f; p.cs[dirBH + (size_t)bglob * H + u] = 0.f; }
-    cluster_sync_all();            // peers' exchange buffers are initialised before anyone stores into them
+    cluster_arrive(); cluster_wait();    // peers' exchange buffers are initialised before anyone stores into them
     for (int j = 0; j < L; ++j) {
         const int t = dir ? L - 1 - j : j;
         const int cur = j & 1, nxt = cur ^ 1;
@@ -133,7 +121,7 @@ __global__ void __launch_bounds__(RT, 1) bilstm_fwd_loop_kernel(const BiLoopArgs
         if (any) {                 // publish this CTA's slice of the new hidden state to every CTA of the cluster
             const uint32_t offb = (uint32_t)(((size_t)nxt * RBG * H + (size_t)cb * H + u) * 4);
             for (int r = 0; r < CS; ++r) st_cluster_f32(peer_addr(hbuf, (uint32_t)r) + offb, hn);
-            cluster_sync_all();
+            cluster_arrive(); cluster_wait();
         }
         // else: the whole group is frozen at this position.  Along a direction's processing order that happens only BEFORE the first valid
         // step (reverse direction: the state is still the zero initial state, which both exchange buffers hold) or AFTER the last one
@@ -171,7 +159,7 @@ __global__ void __launch_bounds__(RT, 1) bilstm_bwd_loop_kernel(const BiLoopArgs
     const int ks = tid >> 5;                           // product role: rows [ks * 4H / 8, (ks + 1) * 4H / 8)
     const size_t dirBH = (size_t)dir * (L + 1) * B * H, dirG = (size_t)dir * L * B * 4 * H;
     float dc_reg = 0.f, dh_rec = 0.f;
-    cluster_sync_all();
+    cluster_arrive(); cluster_wait();
     for (int j = L - 1; j >= 0; --j) {
         const int t = dir ? L - 1 - j : j;
         const int cur = j & 1;
@@ -204,7 +192,7 @@ __global__ void __launch_bounds__(RT, 1) bilstm_bwd_loop_kernel(const BiLoopArgs
                 for (int r = 0; r < CS; ++r) st_cluster_f32(peer_addr(dgb, (uint32_t)r) + offb, d4[g]);
             }
         }
-        cluster_sync_all();
+        cluster_arrive(); cluster_wait();
         if (j > 0) {
             float acc[RBG];
 #pragma unroll

@@ -35,14 +35,19 @@ int check_cuda(cudaError_t e, const char* what, const char* file, int line);
     } while (0)
 
 // Named kernel timers (b200tts_kernel_timing): when enabled, CUDA events are recorded on the launching stream around the dominant kernels;
-// bench.py reads per-name totals after a synchronize.  Disabled (the default) they cost one relaxed load.
+// bench.py reads per-name totals after a synchronize.  Disabled (the default) they cost one relaxed load.  A null name times nothing.
 void ktimer_start(const char* name, cudaStream_t st);
 void ktimer_stop(const char* name, cudaStream_t st);
 struct KernelTimer {
     const char* name; cudaStream_t st;
-    KernelTimer(const char* n, cudaStream_t s) : name(n), st(s) { ktimer_start(n, s); }
-    ~KernelTimer() { ktimer_stop(name, st); }
+    KernelTimer(const char* n, cudaStream_t s) : name(n), st(s) { if (n) ktimer_start(n, s); }
+    ~KernelTimer() { if (name) ktimer_stop(name, st); }
 };
+
+// tcgen05 GEMM (gemm_tc.cu): bf16 tensor maps with SWIZZLE_128B.  map3: dims {d0, d1, d2} (d0 contiguous), byte strides of d1 / d2, box
+// {b0, b1, b2}; mapN: rank <= 5, rank - 1 byte strides
+int tc_make_map3_bf16(void* map, const void* base, int d0, int d1, int d2, size_t stride1, size_t stride2, int b0, int b1, int b2);
+int tc_make_mapN_bf16(void* map, const void* base, int rank, const unsigned long long* dims, const unsigned long long* strides, const unsigned* box);
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 static inline size_t align_up_sz(size_t x, size_t a) { return (x + a - 1) / a * a; }

@@ -16,6 +16,7 @@
 #include <cuda_bf16.h>
 #include <cooperative_groups.h>
 #include "decoder_internal.cuh"
+#include "persist.cuh"
 
 namespace b200tts {
 
@@ -56,65 +57,7 @@ struct LoopArgs {
     long long* prof;                          // optional [gridDim.x][8] per-phase cycle totals (thread 0 of each CTA)
 };
 
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
-
-__device__ __forceinline__ void ldmatrix_x4(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, const void* p) {
-    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(p);
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
-__device__ __forceinline__ uint32_t pack2(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ float tanh_fast(float x) {
-    float y;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-
-// Monotonic-counter grid barrier.  Returns false if the watchdog fired (caller must leave the loop).
-__device__ __forceinline__ bool grid_barrier(unsigned* counter, unsigned& target, unsigned nblocks, int* abort_flag) {
-    __shared__ int s_ok;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += nblocks;
-        // arrival = ONE release-reduction (cumulative over the CTA's writes, which the __syncthreads above made visible to thread 0);
-        // the wait polls with relaxed loads and issues a single acquire fence after the last one
-        asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(counter) : "memory");
-        int ok = 1;
-        const long long t0 = clock64();
-        unsigned polls = 0;
-        for (;;) {
-            unsigned v;
-            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-            if (v >= target) break;
-            if ((++polls & 255u) == 0 && (clock64() - t0 > 4000000000ll || *reinterpret_cast<volatile int*>(abort_flag))) {
-                ok = 0; *abort_flag = 1; break;
-            }
-        }
-        asm volatile("fence.acquire.gpu;" ::: "memory");
-        s_ok = ok;
-    }
-    __syncthreads();
-    return s_ok != 0;
-}
+using namespace tcx;
 
 struct Smem {
     __nv_bfloat16* W;      // [ROWS][Kp + 8]
@@ -127,6 +70,7 @@ struct Smem {
 template <bool ATT, int NSTAGE>
 __global__ void __launch_bounds__(PT, 1) lstm_loop_kernel(const LoopArgs p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ int s_ok;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int cta = blockIdx.x;
     const int rb = cta % p.RB, bh = cta / p.RB;
@@ -164,12 +108,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_loop_kernel(const LoopArgs p) {
     const int nchunks = (Kp + CHUNK - 1) / CHUNK;
     const float inv_h = 1.f / (1.f - p.rate_h), inv_c = 1.f / (1.f - p.rate_c);
     unsigned target = 0;
-    long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    long long prof_t = clock64();
-#define PROF_MARK(slot)                                                      \
-    do {                                                                     \
-        if (p.prof && tid == 0) { const long long now = clock64(); prof_acc[slot] += now - prof_t; prof_t = now; } \
-    } while (0)
+    PROF_DECL
 
     for (int i = 0; i < p.T; ++i) {
         // =================== gate GEMM: acc[b, r] = sum_k act[b, k] * W[r, k] ===================
@@ -350,7 +289,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_loop_kernel(const LoopArgs p) {
             }
         }
         PROF_MARK(2);
-        if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag)) return;
+        if (!grid_barrier<false>(p.barrier, target, nblocks, p.abort_flag, &s_ok)) return;
         PROF_MARK(3);
 
         if (ATT) {
@@ -524,13 +463,11 @@ __global__ void __launch_bounds__(PT, 1) lstm_loop_kernel(const LoopArgs p) {
                 }
             }
             PROF_MARK(6);
-            if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag)) return;
+            if (!grid_barrier<false>(p.barrier, target, nblocks, p.abort_flag, &s_ok)) return;
             PROF_MARK(7);
         }
     }
-    if (p.prof && tid == 0)
-        for (int k = 0; k < 8; ++k) p.prof[(size_t)cta * 8 + k] = prof_acc[k];
-#undef PROF_MARK
+    PROF_FLUSH;
 }
 
 size_t loop_smem_bytes(int Kp, int A, bool att, int L, int M, int nstage) {
@@ -660,19 +597,9 @@ bool persist_supported(const b200tts_decoder_shape& s) {
 
 static int launch_loop(bool att, const LoopArgs& a, size_t smem, cudaStream_t st) {
     void* fn = att ? (void*)lstm_loop_kernel<true, ATT_STAGES> : (void*)lstm_loop_kernel<false, GEN_STAGES>;
-    B200_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PT, smem));
-    int dev = 0, sms = 0;
-    B200_CUDA(cudaGetDevice(&dev));
-    B200_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    const int grid = a.RB * a.NBH;
-    B200_REQUIRE(per_sm * sms >= grid, "persistent loop: %d CTAs cannot be co-resident (%d per SM x %d SMs)", grid, per_sm, sms);
     LoopArgs args = a;
     void* params[] = {&args};
-    B200_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(PT), params, smem, st));
-    B200_LAUNCH_CHECK();
-    return B200TTS_OK;
+    return launch_persistent(fn, a.RB * a.NBH, PT, smem, params, st, "persistent loop", nullptr);
 }
 
 // bf16 memory, Wcomb and the fragment-major projections shared by the forward and backward persistent kernels
@@ -704,9 +631,7 @@ int persist_att_loop(const b200tts_decoder_shape& s, const b200tts_decoder_param
     const int B = s.B, T = s.T, D = s.D, M = s.M, MD = M + D;
     __nv_bfloat16* aib = reinterpret_cast<__nv_bfloat16*>(pws + l.aib);
     __nv_bfloat16* memb = reinterpret_cast<__nv_bfloat16*>(pws + l.memb);
-    unsigned* barrier = reinterpret_cast<unsigned*>(pws + l.barrier);
     B200_CUDA(cudaMemsetAsync(aib, 0, (size_t)B * l.Kp_att * 2, st));                 // operand of step 0
-    B200_CUDA(cudaMemsetAsync(barrier, 0, 256, st));
     __nv_bfloat16* wcb = reinterpret_cast<__nv_bfloat16*>(pws + l.wcb);
     __nv_bfloat16* memTf = reinterpret_cast<__nv_bfloat16*>(pws + l.memTf);
     uint4* memFf = reinterpret_cast<uint4*>(pws + l.memFf);
@@ -722,8 +647,7 @@ int persist_att_loop(const b200tts_decoder_shape& s, const b200tts_decoder_param
     a.Wq = w.attn_query; a.qpart = ws + fl.qpart; a.qsave = ws + fl.q; a.WcB = wcb; a.memTf = memTf; a.MT = l.MT; a.bias = w.attn_bias; a.v = w.attn_energy;
     a.memb = memb; a.ldm = l.ldm; a.memFf = memFf; a.M16 = l.M16; a.lengths = in.text_lengths; a.cum = ws + fl.cum;
     a.align = align; a.align_bstride = (long long)T * s.L;
-    a.barrier = barrier; a.abort_flag = reinterpret_cast<int*>(barrier + 32);
-    a.prof = reinterpret_cast<long long*>(pws + l.barrier + 256);
+    B200_TRY(reset_grid_barrier(pws + l.barrier, a, st));
     return launch_loop(true, a, loop_smem_bytes(l.Kp_att, s.A, true, s.L, M, ATT_STAGES), st);
 }
 
@@ -733,17 +657,15 @@ int persist_gen_loop(const b200tts_decoder_shape& s, const b200tts_decoder_param
     const PersistLayout l = persist_layout(s);
     const int B = s.B, T = s.T, D = s.D;
     __nv_bfloat16* hgb = reinterpret_cast<__nv_bfloat16*>(pws + l.hgb);
-    unsigned* barrier = reinterpret_cast<unsigned*>(pws + l.barrier);
     B200_CUDA(cudaMemsetAsync(hgb, 0, (size_t)(l.Kp_gen != D ? (size_t)(T + 1) : 1) * B * l.Kp_gen * 2, st));
-    B200_CUDA(cudaMemsetAsync(barrier, 0, 256, st));
     LoopArgs a{};
     a.B = B; a.T = T; a.D = D; a.K = D; a.Kp = l.Kp_gen; a.RB = D / UNITS; a.NBH = (B + BT - 1) / BT;
     a.W = w.gen_w_hh; a.ldw = D;
     a.actb = hgb; a.actf = ws + fl.hg; a.ldf = D; a.hcol = 0;
     a.gates = ws + fl.gg; a.cstate = ws + fl.cg;
     a.mask_h = in.mask_gen_h; a.mask_c = in.mask_gen_c; a.kind = s.cell_kind; a.training = s.training; a.rate_h = s.rate_h; a.rate_c = s.rate_c;
-    a.barrier = barrier; a.abort_flag = reinterpret_cast<int*>(barrier + 32);
-    a.prof = reinterpret_cast<long long*>(pws + l.barrier + 256) + 148 * 8;
+    B200_TRY(reset_grid_barrier(pws + l.barrier, a, st));
+    a.prof += 148 * 8;
     return launch_loop(false, a, loop_smem_bytes(l.Kp_gen, s.A, false, 0, 0, GEN_STAGES), st);
 }
 

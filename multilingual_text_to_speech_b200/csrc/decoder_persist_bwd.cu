@@ -13,7 +13,7 @@
 #include <stdlib.h>
 #include <cuda_bf16.h>
 #include "decoder_internal.cuh"
-#include "tc_ptx.cuh"
+#include "persist.cuh"
 
 namespace b200tts {
 
@@ -40,98 +40,12 @@ struct BwdLoopArgs {
     long long* prof;
 };
 
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem));
-}
-__device__ __forceinline__ void cp_async_commit_wait() { asm volatile("cp.async.commit_group;\ncp.async.wait_group 0;\n" ::); }
-__device__ __forceinline__ void ldmatrix_x4(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, const void* p) {
-    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(p);
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void ldmatrix_x4_trans(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, const void* p) {
-    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(p);
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-struct NoOverlap { __device__ __forceinline__ void operator()() const {} };
-// `overlap` runs on every thread BETWEEN the CTA's arrival and its wait: work that does not depend on other CTAs (next step's operand
-// prefetch) hides under the barrier latency instead of delaying the arrival
-template <typename Overlap = NoOverlap>
-__device__ __forceinline__ bool grid_barrier(unsigned* counter, unsigned& target, unsigned nblocks, int* abort_flag, bool async_fence = false,
-                                             Overlap overlap = Overlap()) {
-    __shared__ int s_ok;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += nblocks;
-        if (async_fence) tcx::proxy_fence_global();     // global data written above is read by other CTAs through TMA (async proxy)
-        // arrival = ONE release-reduction (cumulative over the CTA's writes, which the __syncthreads above made visible to thread 0);
-        // the wait polls with relaxed loads and issues a single acquire fence after the last one
-        asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(counter) : "memory");
-    }
-    overlap();
-    if (threadIdx.x == 0) {
-        int ok = 1;
-        const long long t0 = clock64();
-        unsigned polls = 0;
-        for (;;) {
-            unsigned v;
-            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-            if (v >= target) break;
-            if ((++polls & 255u) == 0 && (clock64() - t0 > 4000000000ll || *reinterpret_cast<volatile int*>(abort_flag))) {
-                ok = 0; *abort_flag = 1; break;
-            }
-        }
-        asm volatile("fence.acquire.gpu;" ::: "memory");
-        s_ok = ok;
-    }
-    __syncthreads();
-    return s_ok != 0;
-}
-
-// thread-block cluster (CTA pair) primitives: split arrive / wait barrier and a distributed-shared-memory store
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-__device__ __forceinline__ void st_peer_f32(const float* local_smem, uint32_t peer_rank, float v) {
-    uint32_t ra;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"((uint32_t)__cvta_generic_to_shared(local_smem)), "r"(peer_rank));
-    asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(ra), "f"(v) : "memory");
-}
-__device__ __forceinline__ void l2_prefetch(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-// remote store that completes its 4 bytes on the PEER's mbarrier (data + signal in one instruction): the pair exchanges need no cluster
-// barrier and none of the memory fence its release semantics imply
-__device__ __forceinline__ void st_async_peer_f32(const float* local_smem, const uint64_t* local_bar, uint32_t peer_rank, float v) {
-    uint32_t ra, rb;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"((uint32_t)__cvta_generic_to_shared(local_smem)), "r"(peer_rank));
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rb) : "r"((uint32_t)__cvta_generic_to_shared(local_bar)), "r"(peer_rank));
-    asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(ra), "r"(__float_as_uint(v)), "r"(rb) : "memory");
-}
-// tanh of the recomputed cell state in the reverse loops: the same ex2-based form the forward loops of the bf16 mode use (~1e-6 relative)
-__device__ __forceinline__ float tanh_exp(float x) { return 2.f * __fdividef(1.f, 1.f + __expf(-2.f * x)) - 1.f; }
-
-#define BPROF_DECL long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0}; long long prof_t = clock64();
-#define BPROF_MARK(slot)                                                                                         \
-    do {                                                                                                         \
-        if (p.prof && threadIdx.x == 0) { const long long now = clock64(); prof_acc[slot] += now - prof_t; prof_t = now; } \
-    } while (0)
-#define BPROF_FLUSH                                                                                              \
-    do {                                                                                                         \
-        if (p.prof && threadIdx.x == 0)                                                                          \
-            for (int k9 = 0; k9 < 8; ++k9) p.prof[(size_t)blockIdx.x * 8 + k9] = prof_acc[k9];                   \
-    } while (0)
+using namespace tcx;
 
 // Generator-LSTM reverse loop (no attention): NOUT = D.
 __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_kernel(const BwdLoopArgs p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ int s_ok;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int cta = blockIdx.x;
     const int kb = cta % KB, nb = (cta / KB) % NBK, bh = cta / (KB * NBK);
@@ -160,7 +74,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_kernel(const BwdLoopArgs 
 #pragma unroll
     for (int e = 0; e < MAXE; ++e) { dc_reg[e] = 0.f; dhz_reg[e] = 0.f; }
     unsigned target = 0;
-    BPROF_DECL
+    PROF_DECL
 
     for (int i = p.T - 1; i >= 0; --i) {
         const bool last = (i == p.T - 1);
@@ -209,9 +123,9 @@ __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_kernel(const BwdLoopArgs 
                 }
             }
         }
-        BPROF_MARK(0);
-        if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag)) return;
-        BPROF_MARK(1);
+        PROF_MARK(0);
+        if (!grid_barrier<false>(p.barrier, target, nblocks, p.abort_flag, &s_ok)) return;
+        PROF_MARK(1);
         if (i == 0) break;
 
         // ---------------- P2: partial[kb] = dgates[:, K-block kb] . W[K-block kb, N-block nb] ----------------
@@ -261,7 +175,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_kernel(const BwdLoopArgs 
                         }
             }
         }
-        if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag)) return;
+        if (!grid_barrier<false>(p.barrier, target, nblocks, p.abort_flag, &s_ok)) return;
     }
 }
 
@@ -308,16 +222,6 @@ struct AttBwdArgs {
     long long* prof;
 };
 
-__device__ __forceinline__ uint32_t pack2(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ float tanh_fast(float x) {
-    float y;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-
 // Build the Toeplitz pair arrays of the zero-padded cumulative weights: Ph[x] = (hi[x], hi[x+1]), Pl likewise, where
 // cumpad[j] = cum[j - half] and cum = hi + lo with hi, lo in bf16 (16 mantissa bits in total).
 __device__ __forceinline__ void build_pairs(uint32_t* Ph, uint32_t* Pl, const float* cum, int L, int half, int n, int tid, int nthreads) {
@@ -341,6 +245,7 @@ __global__ void __launch_bounds__(PT, 1) att_bwd_loop_kernel(const __grid_consta
     unsigned char* smem_raw = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw0) + 1023) & ~(uintptr_t)1023);
     __shared__ uint64_t full_bar, accum_bar, xb1, xb2;      // xb1 / xb2: arrival of the peer's softmax dot / query-gradient partial + G halo tile
     __shared__ uint32_t tmem_base_s;
+    __shared__ int s_ok;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int cta = blockIdx.x;
     const int kb = cta % KBA, nb = TC ? cta / KBA : (cta / KBA) % NBA, bh = TC ? 0 : cta / (KBA * NBA);
@@ -422,7 +327,7 @@ __global__ void __launch_bounds__(PT, 1) att_bwd_loop_kernel(const __grid_consta
     float* s_dotx = s_dqx + A;                            // [4]  the peer's partial softmax dot
     float* s_stage = s_dotx + 4;                          // [L16] d cum staging
     uint2* s_bf = reinterpret_cast<uint2*>(s_stage + L16); // [M16][32] B fragments (hi / lo split of d ctx) of the dw product, shared by all warps
-    BPROF_DECL
+    PROF_DECL
 
     const int pc = cta >> 1;
     // cell-backward operands of this thread's (b, u) pairs (owner CTAs): fetched a whole reverse step ahead, at the end of the previous
@@ -592,7 +497,7 @@ __global__ void __launch_bounds__(PT, 1) att_bwd_loop_kernel(const __grid_consta
                 if (l < L) p.de[((size_t)i * B + b) * L + l] = d;
             }
             __syncthreads();
-            BPROF_MARK(0);
+            PROF_MARK(0);
             // energies backward on the tensor cores; warp owns position tiles {warp, warp + 8}
             float dqacc[16][2];
 #pragma unroll
@@ -712,9 +617,9 @@ __global__ void __launch_bounds__(PT, 1) att_bwd_loop_kernel(const __grid_consta
             __syncthreads();
             for (int j = t_lo * 16 + tid; j < t_hi * 16 && j < L; j += PT) dcum[j] = s_stage[j];
         }
-        BPROF_MARK(1);
-        if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag)) break;
-        BPROF_MARK(2);
+        PROF_MARK(1);
+        if (!grid_barrier<false>(p.barrier, target, nblocks, p.abort_flag, &s_ok)) break;
+        PROF_MARK(2);
 
         // =========================== PB: attention-LSTM cell backward ===========================
         if (owner) {
@@ -849,11 +754,11 @@ __global__ void __launch_bounds__(PT, 1) att_bwd_loop_kernel(const __grid_consta
                 }
             }
         }
-        BPROF_MARK(3);
+        PROF_MARK(3);
         // the operands of the next cell backward are fetched between this CTA's arrival and its wait (the compiler parks them in local
         // memory, i.e. the thread waits for the loads right there: under the barrier that wait is free)
-        if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag, TC, [&]() { pb_prefetch(i - 1); })) break;
-        BPROF_MARK(4);
+        if (!grid_barrier<TC>(p.barrier, target, nblocks, p.abort_flag, &s_ok, [&]() { pb_prefetch(i - 1); })) break;
+        PROF_MARK(4);
         if (i == 0) break;
 
         // =========================== P2: [d ctx | d h](i-1) partial = dgates_i[:, kb] . W[kb, nb] ===========================
@@ -950,11 +855,11 @@ __global__ void __launch_bounds__(PT, 1) att_bwd_loop_kernel(const __grid_consta
                         }
             }
         }
-        BPROF_MARK(5);
-        if (!grid_barrier(p.barrier, target, nblocks, p.abort_flag)) break;
-        BPROF_MARK(6);
+        PROF_MARK(5);
+        if (!grid_barrier<false>(p.barrier, target, nblocks, p.abort_flag, &s_ok)) break;
+        PROF_MARK(6);
     }
-    BPROF_FLUSH;
+    PROF_FLUSH;
     if (TC) {
         tcx::tc_fence_before();
         __syncthreads();
@@ -1284,8 +1189,6 @@ static bool att_bwd_pick(const b200tts_decoder_shape& s, AttBwdGeom* out) {
 bool persist_att_bwd_supported(const b200tts_decoder_shape& s) { return att_bwd_pick(s, nullptr); }
 bool persist_att_bwd_tc(const b200tts_decoder_shape& s) { AttBwdGeom g{}; return att_bwd_pick(s, &g) && g.tc; }
 
-int tc_make_mapN_bf16(void* map, const void* base, int rank, const unsigned long long* dims, const unsigned long long* strides, const unsigned* box);
-
 int persist_att_bwd_loop(const b200tts_decoder_shape& s, const b200tts_decoder_params& w, const b200tts_decoder_inputs& in,
                          const DecoderLayout& fl, const float* fws, const PersistLayout& pl, const unsigned char* pws,
                          const float* align, const float* dalign, const float* dh_static, const float* dctx_static, float* dgates,
@@ -1318,22 +1221,14 @@ int persist_att_bwd_loop(const b200tts_decoder_shape& s, const b200tts_decoder_p
     a.memFb = reinterpret_cast<const uint4*>(pws + pl.memFb); a.M16 = pl.M16;
     a.dqp_after_g = 1;
     a.lengths = in.text_lengths; a.dctx_tot = dctx_tot; a.dq = dq; a.de = reinterpret_cast<float*>(extra + x.de);
-    a.barrier = reinterpret_cast<unsigned*>(extra + x.barrier); a.abort_flag = reinterpret_cast<int*>(a.barrier + 32);
-    a.prof = reinterpret_cast<long long*>(extra + x.barrier + 256);
     const float* wcombT = reinterpret_cast<const float*>(pws + pl.wcombT);
-    B200_CUDA(cudaMemsetAsync(a.barrier, 0, 256, st));
+    B200_TRY(reset_grid_barrier(extra + x.barrier, a, st));
     att_bwd_prep_kernel<<<148 * 4, 256, 0, st>>>(wcb, wcb2, memTf, wcombT, fws + fl.memT, B, L, A, s.K, x.MT);
     B200_LAUNCH_CHECK();
-    const size_t smem = geo.smem;
     void* fn = geo.tc ? (geo.UN == TUN ? (void*)att_bwd_loop_kernel<true, TUN> : (void*)att_bwd_loop_kernel<true, TUN_WIDE>)
                       : (void*)att_bwd_loop_kernel<false, 0>;
-    B200_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = geo.grid;
-    int per_sm = 0, dev = 0, sms = 0;
-    B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PT, smem));
-    B200_CUDA(cudaGetDevice(&dev));
-    B200_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    B200_REQUIRE(per_sm * sms >= grid && grid % 2 == 0 && grid / 2 >= B, "persistent attention backward: %d CTAs cannot be co-resident / paired", grid);
+    B200_REQUIRE(grid % 2 == 0 && grid / 2 >= B, "persistent attention backward: %d CTAs cannot be paired", grid);
     CUtensorMap tm;
     memset(&tm, 0, sizeof(tm));
     if (geo.tc) {
@@ -1345,24 +1240,8 @@ int persist_att_bwd_loop(const b200tts_decoder_shape& s, const b200tts_decoder_p
         B200_TRY(tc_make_mapN_bf16(&tm, a.dgb, 5, dims, strides, box));
     }
     void* params[] = {&tm, &a};
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(PT); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attrs[2];
-    attrs[0].id = cudaLaunchAttributeCooperative;
-    // profiling aid: ncu cannot capture a launch that is BOTH cooperative and clustered; the kernel carries its own grid barrier, so on an
-    // otherwise idle GPU (all CTAs resident: <= 148, one per SM) the cooperative attribute can be dropped for a capture
-    attrs[0].val.cooperative = getenv("B200TTS_PROFILE_NO_COOP") ? 0 : 1;
-    attrs[1].id = cudaLaunchAttributeClusterDimension;          // the attention backward of an utterance runs on a CTA pair
-    attrs[1].val.clusterDim.x = 2; attrs[1].val.clusterDim.y = 1; attrs[1].val.clusterDim.z = 1;
-    cfg.attrs = attrs; cfg.numAttrs = 2;
-    int nclusters = 0;
-    B200_CUDA(cudaOccupancyMaxActiveClusters(&nclusters, fn, &cfg));
-    B200_REQUIRE(nclusters * 2 >= grid, "persistent attention backward: only %d CTA pairs can be co-resident, %d needed", nclusters, grid / 2);
-    {
-        KernelTimer kt("att_bwd_loop_kernel", st);
-        B200_CUDA(cudaLaunchKernelExC(&cfg, fn, params));
-    }
-    B200_LAUNCH_CHECK();
+    // the attention backward of an utterance runs on a CTA pair
+    B200_TRY(launch_persistent(fn, grid, PT, geo.smem, params, st, "persistent attention backward", "att_bwd_loop_kernel", 2, true));
     // parallel post pass
     AttPostArgs pp{};
     pp.B = B; pp.T = T; pp.L = L; pp.A = A; pp.KC = s.K; pp.MT = x.MT;
@@ -1407,27 +1286,13 @@ int persist_gen_bwd_loop(const b200tts_decoder_shape& s, const b200tts_decoder_p
     size_t off = 0;
     a.dgb = reinterpret_cast<__nv_bfloat16*>(extra + off); off += ((size_t)B * 4 * D * 2 + 255) / 256 * 256;
     a.part = reinterpret_cast<float*>(extra + off); off += ((size_t)KB * B * D * 4 + 255) / 256 * 256;
-    a.barrier = reinterpret_cast<unsigned*>(extra + off);
-    a.abort_flag = reinterpret_cast<int*>(a.barrier + 32);
-    a.prof = reinterpret_cast<long long*>(extra + off + 256);
     a.hcol = 0;
-    B200_CUDA(cudaMemsetAsync(a.barrier, 0, 256, st));
+    B200_TRY(reset_grid_barrier(extra + off, a, st));
     const size_t smem = ((size_t)4 * a.UK * (a.UN + 8) + (size_t)BT * (4 * a.UK + 8)) * 2;
     B200_REQUIRE(smem <= 227 * 1024, "persistent backward: %zu B of shared memory needed", smem);
-    void* fn = (void*)lstm_bwd_loop_kernel;
-    B200_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int grid = KB * NBK * a.NBH;
-    int per_sm = 0, dev = 0, sms = 0;
-    B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PT, smem));
-    B200_CUDA(cudaGetDevice(&dev));
-    B200_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    B200_REQUIRE(per_sm * sms >= grid, "persistent backward: %d CTAs cannot be co-resident", grid);
     void* params[] = {&a};
-    {
-        KernelTimer kt("lstm_bwd_loop_kernel", st);
-        B200_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(PT), params, smem, st));
-    }
-    B200_LAUNCH_CHECK();
+    B200_TRY(launch_persistent((void*)lstm_bwd_loop_kernel, KB * NBK * a.NBH, PT, smem, params, st, "persistent backward",
+                               "lstm_bwd_loop_kernel"));
     return B200TTS_OK;
 }
 

@@ -14,10 +14,9 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include "decoder_internal.cuh"
+#include "persist.cuh"
 
 namespace b200tts {
-
-int tc_make_map3_bf16(void* map, const void* base, int d0, int d1, int d2, size_t stride1, size_t stride2, int b0, int b1, int b2);
 
 namespace {
 
@@ -47,117 +46,7 @@ struct TcBwdArgs {
     long long* prof;
 };
 
-// ------------------------------------------------------------------------------------------------
-// PTX wrappers
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    const uint32_t addr = smem_u32(bar);
-    const long long t0 = clock64();
-    for (;;) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(addr), "r"(parity)
-            : "memory");
-        if (done) return;
-        if (clock64() - t0 > 4000000000ll) __trap();       // ~2 s: a protocol bug must not hang the GPU
-    }
-}
-__device__ __forceinline__ void tma_load_3d(void* smem, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(smem_u32(smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence_shared() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void l2_prefetch(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-// tanh of the recomputed cell state in the reverse loops: the same ex2-based form the forward loops of the bf16 mode use (~1e-6 relative)
-__device__ __forceinline__ float tanh_exp(float x) { return 2.f * __fdividef(1.f, 1.f + __expf(-2.f * x)) - 1.f; }
-// thread-block cluster (CTA pair) primitives: split arrive / wait barrier and a distributed-shared-memory store
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-__device__ __forceinline__ void st_peer_f32(const float* local_smem, uint32_t peer_rank, float v) {
-    uint32_t ra;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(local_smem)), "r"(peer_rank));
-    asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(ra), "f"(v) : "memory");
-}
-// named barrier among the compute warps only
-__device__ __forceinline__ void csync() { asm volatile("bar.sync 1, %0;" ::"n"(CT) : "memory"); }
-
-// K-major SWIZZLE_128B operand tile (rows of 64 bf16 = 128 B, 8-row groups 1024 B apart): UMMA shared-memory descriptor
-__device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)1 << 16;
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-
-
-
-__device__ __forceinline__ bool grid_barrier(unsigned* counter, unsigned& target, unsigned nblocks, int* abort_flag, int* s_ok) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += nblocks;
-        proxy_fence_global();          // the bf16 gate gradients written above are read by other CTAs through TMA (async proxy)
-        asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(counter) : "memory");
-        int ok = 1;
-        const long long t0 = clock64();
-        unsigned polls = 0;
-        for (;;) {
-            unsigned v;
-            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-            if (v >= target) break;
-            if ((++polls & 255u) == 0 && (clock64() - t0 > 4000000000ll || *reinterpret_cast<volatile int*>(abort_flag))) {
-                ok = 0; *abort_flag = 1; break;
-            }
-        }
-        asm volatile("fence.acquire.gpu;" ::: "memory");
-        *s_ok = ok;
-    }
-    __syncthreads();
-    return *s_ok != 0;
-}
+using namespace tcx;
 
 __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_tc_kernel(const __grid_constant__ CUtensorMap tmG, const TcBwdArgs p) {
     extern __shared__ __align__(1024) unsigned char smem_raw0[];
@@ -245,12 +134,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_tc_kernel(const __grid_co
 
     unsigned target = 0;
     uint32_t it = 0;                         // products done (mbarrier phase)
-    long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    long long prof_t = clock64();
-#define PROF_MARK(slot)                                                      \
-    do {                                                                     \
-        if (p.prof && tid == 0) { const long long now = clock64(); prof_acc[slot] += now - prof_t; prof_t = now; } \
-    } while (0)
+    PROF_DECL
 
     for (int i = p.T - 1; i >= 0; --i) {
         const bool last = (i == p.T - 1);
@@ -299,7 +183,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_tc_kernel(const __grid_co
             }
         }
         PROF_MARK(0);
-        if (!grid_barrier(bar_counter, target, nblocks, p.abort_flag, &s_ok)) break;
+        if (!grid_barrier<true>(bar_counter, target, nblocks, p.abort_flag, &s_ok)) break;
         PROF_MARK(1);
         if (i == 0) break;
 
@@ -345,12 +229,10 @@ __global__ void __launch_bounds__(PT, 1) lstm_bwd_loop_tc_kernel(const __grid_co
         }
         ++it;
         PROF_MARK(3);
-        if (!grid_barrier(bar_counter, target, nblocks, p.abort_flag, &s_ok)) break;
+        if (!grid_barrier<true>(bar_counter, target, nblocks, p.abort_flag, &s_ok)) break;
         PROF_MARK(4);
     }
-    if (p.prof && tid == 0)
-        for (int k = 0; k < 8; ++k) p.prof[(size_t)cta * 8 + k] = prof_acc[k];
-#undef PROF_MARK
+    PROF_FLUSH;
     tc_fence_before();
     __syncthreads();
     if (warp == NCW + 1) {
@@ -386,25 +268,13 @@ int tc_persist_gen_bwd_loop(const b200tts_decoder_shape& s, const b200tts_decode
     a.dgb_step = dgb_hist ? (long long)B * 4 * D : 0; a.dgb_rows = dgb_hist ? B : 0;
     off += ((size_t)B * 4 * D * 2 + 255) / 256 * 256;
     a.part = reinterpret_cast<float*>(extra + off); off += ((size_t)8 * B * D * 4 + 255) / 256 * 256;
-    a.barrier = reinterpret_cast<unsigned*>(extra + off);
-    a.abort_flag = reinterpret_cast<int*>(a.barrier + 32);
-    a.prof = reinterpret_cast<long long*>(extra + off + 256);
-    B200_CUDA(cudaMemsetAsync(a.barrier, 0, 256, st));
+    B200_TRY(reset_grid_barrier(extra + off, a, st));
     CUtensorMap tm;        // {64 columns, B rows, 4D/64 k-blocks}: k-block stride 128 B, row stride 4D * 2 B
     B200_TRY(tc_make_map3_bf16(&tm, a.dgb, KB, dgb_hist ? s.T * B : B, 4 * D / KB, (size_t)4 * D * 2, 128, KB, BT, a.NNB));
     const size_t smem = bwd_tc_smem_bytes(D);
-    void* fn = (void*)lstm_bwd_loop_tc_kernel;
-    B200_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int grid = NG * a.NNB * a.NBH;
-    int per_sm = 0, dev = 0, sms = 0;
-    B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PT, smem));
-    B200_CUDA(cudaGetDevice(&dev));
-    B200_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    B200_REQUIRE(per_sm * sms >= grid, "tcgen05 persistent backward: %d CTAs cannot be co-resident", grid);
     void* params[] = {&tm, &a};
-    KernelTimer kt("lstm_bwd_loop_tc_kernel", st);
-    B200_CUDA(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(PT), params, smem, st));
-    B200_LAUNCH_CHECK();
+    B200_TRY(launch_persistent((void*)lstm_bwd_loop_tc_kernel, NG * a.NNB * a.NBH, PT, smem, params, st, "tcgen05 persistent backward",
+                               "lstm_bwd_loop_tc_kernel"));
     return B200TTS_OK;
 }
 

@@ -19,11 +19,9 @@
 #include <stdlib.h>
 #include <cuda_bf16.h>
 #include "decoder_internal.cuh"
+#include "persist.cuh"
 
 namespace b200tts {
-
-// gemm_tc.cu: 3-D bf16 tensor map, dims {d0, d1, d2} (d0 contiguous), byte strides of d1 / d2, box {b0, b1, b2}, SWIZZLE_128B
-int tc_make_map3_bf16(void* map, const void* base, int d0, int d1, int d2, size_t stride1, size_t stride2, int b0, int b1, int b2);
 
 namespace {
 
@@ -65,125 +63,10 @@ struct TcLoopArgs {
     long long* prof2;                         // [grid][8] MMA issuer (0-3) / TMA producer (4-7) waits
 };
 
-// ------------------------------------------------------------------------------------------------
-// PTX wrappers
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    const uint32_t addr = smem_u32(bar);
-    const long long t0 = clock64();
-    for (;;) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(addr), "r"(parity)
-            : "memory");
-        if (done) return;
-        if (clock64() - t0 > 4000000000ll) __trap();       // ~2 s: a protocol bug must not hang the GPU
-    }
-}
-__device__ __forceinline__ void tma_load_3d(void* smem, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(smem_u32(smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence_global() { asm volatile("fence.proxy.async.global;" ::: "memory"); }
-__device__ __forceinline__ void proxy_fence_shared() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void l2_prefetch(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-// thread-block cluster (CTA pair) primitives: split arrive / wait barrier and a distributed-shared-memory store
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-__device__ __forceinline__ void st_peer_f32(const float* local_smem, uint32_t peer_rank, float v) {
-    uint32_t ra;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(local_smem)), "r"(peer_rank));
-    asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(ra), "f"(v) : "memory");
-}
-// remote store that completes bytes on the PEER's mbarrier: data + signal in one instruction, no cluster barrier (and none of the memory
-// fence its release semantics imply) on the exchange path
-__device__ __forceinline__ void st_async_peer_f32(const float* local_smem, const uint64_t* local_bar, uint32_t peer_rank, float v) {
-    uint32_t ra, rb;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(smem_u32(local_smem)), "r"(peer_rank));
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rb) : "r"(smem_u32(local_bar)), "r"(peer_rank));
-    asm volatile("st.async.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(ra), "r"(__float_as_uint(v)), "r"(rb) : "memory");
-}
+using namespace tcx;
+
 // named barrier among the compute warps only
 __device__ __forceinline__ void csync() { asm volatile("bar.sync 1, %0;" ::"n"(CT) : "memory"); }
-
-// K-major SWIZZLE_128B operand tile (rows of 64 bf16 = 128 B, 8-row groups 1024 B apart): UMMA shared-memory descriptor
-__device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)1 << 16;
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-
-__device__ __forceinline__ void ldmatrix_x4(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, const void* p) {
-    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(p);
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ unsigned ld_acquire(const unsigned* p) {
-    unsigned v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];\n" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ uint32_t pack2(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ float tanh_fast(float x) {
-    float y;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-    return y;
-}
-
-// gate nonlinearities of the bf16 perf mode: ex2-based, ~1e-6 relative error (the operands of the products are bf16 anyway)
-__device__ __forceinline__ float sigmoid_fast(float x) { return __fdividef(1.f, 1.f + __expf(-x)); }
-__device__ __forceinline__ float tanh_exp(float x) { return 2.f * __fdividef(1.f, 1.f + __expf(-2.f * x)) - 1.f; }
 
 // Block-wide max / sum among the CT compute threads (named barrier 1); `scratch` holds >= 33 floats.
 __device__ __forceinline__ float cblock_max(float v, float* scratch) {
@@ -207,40 +90,6 @@ __device__ __forceinline__ float cblock_sum(float v, float* scratch) {
 #pragma unroll
     for (int o = NCW / 2; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
     return t;
-}
-
-// Monotonic-counter grid barrier over ALL threads of every CTA.  Returns false if the watchdog fired.
-// Arrival is ONE release-reduction (cumulative: it orders the whole CTA's writes, which the preceding __syncthreads made
-// visible to thread 0); the wait polls with relaxed loads and issues a single acquire fence after the last one.
-struct NoOverlap { __device__ __forceinline__ void operator()() const {} };
-// `overlap` runs on every thread BETWEEN the CTA's arrival and its wait: work that does not depend on other CTAs (next step's operand
-// prefetch) hides under the barrier latency instead of delaying the arrival
-template <typename Overlap = NoOverlap>
-__device__ __forceinline__ bool grid_barrier(unsigned* counter, unsigned& target, unsigned nblocks, int* abort_flag, int* s_ok, Overlap overlap = Overlap()) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        target += nblocks;
-        proxy_fence_global();          // the bf16 operand rows written above are read by other CTAs through TMA (async proxy)
-        asm volatile("red.release.gpu.global.add.u32 [%0], 1;" ::"l"(counter) : "memory");
-    }
-    overlap();
-    if (threadIdx.x == 0) {
-        int ok = 1;
-        const long long t0 = clock64();
-        unsigned polls = 0;
-        for (;;) {                      // nothing but the counter load in the polling loop: its round trip is the barrier latency
-            unsigned v;
-            asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-            if (v >= target) break;
-            if ((++polls & 255u) == 0 && (clock64() - t0 > 4000000000ll || *reinterpret_cast<volatile int*>(abort_flag))) {
-                ok = 0; *abort_flag = 1; break;
-            }
-        }
-        asm volatile("fence.acquire.gpu;" ::: "memory");
-        *s_ok = ok;
-    }
-    __syncthreads();
-    return *s_ok != 0;
 }
 
 // ALIAS (large memory dims only): the accumulator staging lives in the TMA slot and the ctx part arrives in p.n_c TMA instructions; the
@@ -421,12 +270,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_loop_tc_kernel(const __grid_consta
     }
     const float inv_h = 1.f / (1.f - p.rate_h), inv_c = 1.f / (1.f - p.rate_c);
     unsigned target = 0;
-    long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    long long prof_t = clock64();
-#define PROF_MARK(slot)                                                      \
-    do {                                                                     \
-        if (p.prof && tid == 0) { const long long now = clock64(); prof_acc[slot] += now - prof_t; prof_t = now; } \
-    } while (0)
+    PROF_DECL
 
     // prologue: the h part of step 0 (operand row 0 is all zeros)
     if (is_producer) produce(0, 1);
@@ -580,7 +424,7 @@ __global__ void __launch_bounds__(PT, 1) lstm_loop_tc_kernel(const __grid_consta
         }
         PROF_MARK(1);
         if (ALIAS) proxy_fence_shared();             // generic-proxy accesses of the staging precede the TMA writes that follow the barrier
-        if (!grid_barrier(bar_counter, target, nblocks, p.abort_flag, &s_ok)) { alive = false; break; }
+        if (!grid_barrier<true>(bar_counter, target, nblocks, p.abort_flag, &s_ok)) { alive = false; break; }
         PROF_MARK(2);
 
         // =================== h part of step i+1: TMA + tcgen05 run while the attention of step i is computed ===================
@@ -850,15 +694,13 @@ __global__ void __launch_bounds__(PT, 1) lstm_loop_tc_kernel(const __grid_consta
             }
             PROF_MARK(6);
             // next step's epilogue operands (L2 hits: prefetched a step ago) are requested between the arrival and the wait
-            if (!grid_barrier(bar_counter, target, nblocks, p.abort_flag, &s_ok, [&]() { if (compute && i + 1 < p.T) prefetch(i + 1, false); })) {
+            if (!grid_barrier<true>(bar_counter, target, nblocks, p.abort_flag, &s_ok, [&]() { if (compute && i + 1 < p.T) prefetch(i + 1, false); })) {
                 alive = false; break;
             }
             PROF_MARK(7);
         }
     }
-    if (p.prof && tid == 0)
-        for (int k = 0; k < 8; ++k) p.prof[(size_t)cta * 8 + k] = prof_acc[k];
-#undef PROF_MARK
+    PROF_FLUSH;
     if (p.prof2 && (is_mma || is_producer) && lane == 0)
         for (int k = 0; k < 4; ++k) p.prof2[(size_t)cta * 8 + (is_producer ? 4 : 0) + k] = rp[k];
     tc_fence_before();
@@ -932,38 +774,15 @@ bool tc_persist_supported(const b200tts_decoder_shape& s) {
 
 static int launch_tc_loop(bool att, const TcLoopArgs& a, const CUtensorMap& tmH, const CUtensorMap& tmC, size_t smem, cudaStream_t st) {
     void* fn = att ? (a.alias_sum ? (void*)lstm_loop_tc_kernel<true, true> : (void*)lstm_loop_tc_kernel<true, false>) : (void*)lstm_loop_tc_kernel<false, false>;
-    B200_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int grid = a.RB * a.NBH;
     TcLoopArgs args = a;
     CUtensorMap mapH = tmH, mapC = tmC;
     void* params[] = {&mapH, &mapC, &args};
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(PT); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-    cudaLaunchAttribute attrs[2];
-    attrs[0].id = cudaLaunchAttributeCooperative;
-    // profiling aid: ncu cannot capture a launch that is BOTH cooperative and clustered; the kernel carries its own grid barrier, so on an
-    // otherwise idle GPU (all CTAs resident: <= 148, one per SM) the cooperative attribute can be dropped for a capture
-    attrs[0].val.cooperative = getenv("B200TTS_PROFILE_NO_COOP") ? 0 : 1;
-    cfg.attrs = attrs; cfg.numAttrs = 1;
     if (att) {      // the attention runs on CTA pairs: clusters of 2 (distributed shared memory + cluster barrier)
         B200_REQUIRE(grid % 2 == 0 && grid / 2 >= a.B, "tcgen05 attention loop: %d CTAs cannot form %d pairs", grid, a.B);
-        attrs[1].id = cudaLaunchAttributeClusterDimension;
-        attrs[1].val.clusterDim.x = 2; attrs[1].val.clusterDim.y = 1; attrs[1].val.clusterDim.z = 1;
-        cfg.numAttrs = 2;
-        int nclusters = 0;
-        B200_CUDA(cudaOccupancyMaxActiveClusters(&nclusters, fn, &cfg));
-        B200_REQUIRE(nclusters * 2 >= grid, "tcgen05 attention loop: only %d CTA pairs can be co-resident, %d needed", nclusters, grid / 2);
-    } else {
-        int per_sm = 0, dev = 0, sms = 0;
-        B200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, PT, smem));
-        B200_CUDA(cudaGetDevice(&dev));
-        B200_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        B200_REQUIRE(per_sm * sms >= grid, "tcgen05 persistent loop: %d CTAs cannot be co-resident (%d per SM x %d SMs)", grid, per_sm, sms);
+        return launch_persistent(fn, grid, PT, smem, params, st, "tcgen05 attention loop", "lstm_loop_tc_kernel<att>", 2, true);
     }
-    KernelTimer kt(att ? "lstm_loop_tc_kernel<att>" : "lstm_loop_tc_kernel<gen>", st);
-    B200_CUDA(cudaLaunchKernelExC(&cfg, fn, params));
-    B200_LAUNCH_CHECK();
-    return B200TTS_OK;
+    return launch_persistent(fn, grid, PT, smem, params, st, "tcgen05 persistent loop", "lstm_loop_tc_kernel<gen>", 1, true);
 }
 
 // Attention-LSTM + attention loop (all T steps).  Expects: ga = input projection, ai row 0 = 0, ca row 0 = 0, cum row 0 = 0,
@@ -974,10 +793,8 @@ int tc_persist_att_loop(const b200tts_decoder_shape& s, const b200tts_decoder_pa
     const TcPersistGeom g = tc_persist_geom(s);
     const int B = s.B, T = s.T, D = s.D, M = s.M, MD = M + D;
     __nv_bfloat16* aib = reinterpret_cast<__nv_bfloat16*>(pws + l.aib);
-    unsigned* barrier = reinterpret_cast<unsigned*>(pws + l.barrier);
     // operand of step 0 and the zero padding columns [MD, Kp)
     B200_CUDA(cudaMemsetAsync(aib, 0, (size_t)(g.Kp_att != MD ? (size_t)(T + 1) : 1) * B * g.Kp_att * 2, st));   // step 0 + padding
-    B200_CUDA(cudaMemsetAsync(barrier, 0, 256, st));
     CUtensorMap tmH, tmC;       // {64 columns, rows, k-block}: k-block stride 128 B, row stride Kp * 2 B
     B200_TRY(tc_make_map3_bf16(&tmH, aib, KB, (T + 1) * B, g.nkb_att, (size_t)g.Kp_att * 2, 128, KB, BT, g.ch_h_att));
     B200_TRY(tc_make_map3_bf16(&tmC, aib, KB, (T + 1) * B, g.nkb_att, (size_t)g.Kp_att * 2, 128, KB, BT, g.ch_c_att));
@@ -998,8 +815,7 @@ int tc_persist_att_loop(const b200tts_decoder_shape& s, const b200tts_decoder_pa
     a.memFf = reinterpret_cast<const uint4*>(pws + l.memFf); a.M16 = l.M16;
     a.lengths = in.text_lengths; a.cum = ws + fl.cum;
     a.align = align; a.align_bstride = (long long)T * s.L;
-    a.barrier = barrier; a.abort_flag = reinterpret_cast<int*>(barrier + 32);
-    a.prof = reinterpret_cast<long long*>(pws + l.barrier + 256);
+    B200_TRY(reset_grid_barrier(pws + l.barrier, a, st));
     a.prof2 = a.prof + 2 * 148 * 8;
     size_t smem = tc_loop_smem_bytes(g.nkb_att, a.slot_kb, s.A, true, s.L, g.alias_att != 0);
     const size_t tab = (size_t)l.MT * 32 * 8;          // shared B-fragment table of the context product, when it fits behind the scratch
@@ -1015,9 +831,7 @@ int tc_persist_gen_loop(const b200tts_decoder_shape& s, const b200tts_decoder_pa
     const TcPersistGeom g = tc_persist_geom(s);
     const int B = s.B, T = s.T, D = s.D;
     __nv_bfloat16* hgb = reinterpret_cast<__nv_bfloat16*>(pws + l.hgb);
-    unsigned* barrier = reinterpret_cast<unsigned*>(pws + l.barrier);
     B200_CUDA(cudaMemsetAsync(hgb, 0, (size_t)(g.Kp_gen != D ? (size_t)(T + 1) : 1) * B * g.Kp_gen * 2, st));
-    B200_CUDA(cudaMemsetAsync(barrier, 0, 256, st));
     CUtensorMap tmH;
     B200_TRY(tc_make_map3_bf16(&tmH, hgb, KB, (T + 1) * B, g.nkb_gen, (size_t)g.Kp_gen * 2, 128, KB, BT, g.ch_h_gen));
     TcLoopArgs a{};
@@ -1027,8 +841,8 @@ int tc_persist_gen_loop(const b200tts_decoder_shape& s, const b200tts_decoder_pa
     a.actb = hgb; a.actf = ws + fl.hg; a.ldf = D; a.hcol = 0;
     a.gates = ws + fl.gg; a.cstate = ws + fl.cg;
     a.mask_h = in.mask_gen_h; a.mask_c = in.mask_gen_c; a.kind = s.cell_kind; a.training = s.training; a.rate_h = s.rate_h; a.rate_c = s.rate_c;
-    a.barrier = barrier; a.abort_flag = reinterpret_cast<int*>(barrier + 32);
-    a.prof = reinterpret_cast<long long*>(pws + l.barrier + 256) + 148 * 8;
+    B200_TRY(reset_grid_barrier(pws + l.barrier, a, st));
+    a.prof += 148 * 8;
     a.prof2 = a.prof + 2 * 148 * 8;
     return launch_tc_loop(false, a, tmH, tmH, tc_loop_smem_bytes(g.nkb_gen, a.slot_kb, s.A, false, 0), st);
 }

@@ -4,6 +4,7 @@
 // 128x128x32 CTA tile, 8 warps (2 x 4), each warp 64x32 through mma.sync.m16n8k16 fed by ldmatrix.
 #include <cuda_bf16.h>
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace b200tts {
 
@@ -21,10 +22,7 @@ struct KernelArgs {
     long long strideA, strideB, strideC;
 };
 
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
+using namespace tcx;
 
 // Stage a 128 x 32 operand tile: global fp32 -> registers (16 floats / thread).
 //   kcontig: element (r, k) at base[r*ld + k]; else at base[k*ld + r].
@@ -74,8 +72,8 @@ __device__ __forceinline__ void tile_store(__nv_bfloat16* sm, bool kcontig, bool
             if (kcontig) {
                 const int r = v >> 3, kq = v & 7;
                 uint2 w;
-                w.x = pack_bf16(regs[j * 4 + 0], regs[j * 4 + 1]);
-                w.y = pack_bf16(regs[j * 4 + 2], regs[j * 4 + 3]);
+                w.x = pack2(regs[j * 4 + 0], regs[j * 4 + 1]);
+                w.y = pack2(regs[j * 4 + 2], regs[j * 4 + 3]);
                 *reinterpret_cast<uint2*>(sm + r * LDS + kq * 4) = w;
             } else {
                 const int k = v >> 5, r4 = v & 31;
@@ -91,16 +89,6 @@ __device__ __forceinline__ void tile_store(__nv_bfloat16* sm, bool kcontig, bool
             else sm[(idx & 127) * LDS + (idx >> 7)] = __float2bfloat16_rn(regs[j]);
         }
     }
-}
-
-__device__ __forceinline__ void ldmatrix_x4(uint32_t& r0, uint32_t& r1, uint32_t& r2, uint32_t& r3, const void* p) {
-    const uint32_t addr = (uint32_t)__cvta_generic_to_shared(p);
-    asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0,%1,%2,%3}, [%4];\n" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-}
-__device__ __forceinline__ void mma_bf16(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};\n"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
 __global__ void __launch_bounds__(NT) gemm_bf16_kernel(const KernelArgs p) {

@@ -15,6 +15,7 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include "common.cuh"
+#include "ptx.cuh"
 
 namespace b200tts {
 
@@ -28,87 +29,7 @@ constexpr int TMEM_COLS = 128;
 constexpr int STG_LD = TBN + 4;                             // fp32 row stride of the epilogue staging tile (16-byte aligned, conflict-free)
 static_assert(4 * 32 * STG_LD * 4 <= STAGES * STAGE_BYTES, "epilogue staging must fit in the operand ring");
 
-// ------------------------------------------------------------------------------------------------
-// PTX wrappers
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    const uint32_t addr = smem_u32(bar);
-    const long long t0 = clock64();
-    for (;;) {
-        uint32_t done;
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(addr), "r"(parity)
-            : "memory");
-        if (done) return;
-        if (clock64() - t0 > 4000000000ll) __trap();       // ~2 s: a protocol bug must not hang the GPU
-    }
-}
-__device__ __forceinline__ void tma_load_3d(void* smem, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(smem_u32(smem)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-          "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]),
-          "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
-          "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-// K-major, 128-byte swizzled operand tile (rows of 64 bf16 = 128 B, 8-row groups 1024 B apart): UMMA shared-memory descriptor
-// (cute::UMMA::SmemDescriptor: start >> 4 | LBO << 16 | SBO << 32 | version 1 << 46 | SWIZZLE_128B (2) << 61)
-__device__ __forceinline__ uint64_t make_sw128_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)1 << 16;                 // leading byte offset (unused for swizzled K-major; canonical value 1)
-    d |= (uint64_t)(1024 >> 4) << 32;       // stride byte offset: next 8-row group
-    d |= (uint64_t)1 << 46;                 // descriptor version (Blackwell)
-    d |= (uint64_t)2 << 61;                 // SWIZZLE_128B
-    return d;
-}
-
-// MN-major, 128-byte swizzled operand tile: 64-element (128 B) lines along MN, one line per k row, 8-row groups 1024 B apart (stride
-// byte offset), the next 64-element MN chunk 8 KB further (leading byte offset); a K = 16 instruction step advances 16 rows = 2048 B
-// (canonical layout Swizzle<3,4,3> o ((8,n),(8,k)):((1,LBO),(8,SBO)) in 16-byte units, cute::UMMA::make_umma_desc<Major::MN>)
-__device__ __forceinline__ uint64_t make_sw128_mn_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)(8192 >> 4) << 16;       // leading byte offset: next 64-wide MN chunk
-    d |= (uint64_t)(1024 >> 4) << 32;       // stride byte offset: next group of 8 k rows
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
+using namespace tcx;
 
 struct TcArgs {
     float* C; const float* bias;
@@ -268,10 +189,6 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 // operand packing: fp32 (either orientation) -> bf16 [batch][rows][Kp], K contiguous, Kp % 8 == 0
 // ------------------------------------------------------------------------------------------------
 // Thread = 8 consecutive k of one row -> ONE 16-byte store (Kp % 8 == 0); rows ride on blockIdx.y: no per-element 64-bit division.
-__device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
 __global__ void pack_kcontig_kernel(__nv_bfloat16* __restrict__ dst, const float* __restrict__ src, int ld, long long bstride, int rows,
                                     int K, int Kp, int kin, long long kos) {
     const float* s = src + (size_t)blockIdx.z * bstride;
@@ -296,7 +213,7 @@ __global__ void pack_kcontig_kernel(__nv_bfloat16* __restrict__ dst, const float
                     }
                 }
             }
-            *reinterpret_cast<uint4*>(drow + k) = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+            *reinterpret_cast<uint4*>(drow + k) = make_uint4(pack2(v[0], v[1]), pack2(v[2], v[3]), pack2(v[4], v[5]), pack2(v[6], v[7]));
         }
     }
 }
@@ -316,7 +233,7 @@ __global__ void pack_transpose_kernel(__nv_bfloat16* __restrict__ dst, const flo
     for (int j = threadIdx.y; j < 32; j += blockDim.y) {
         const int r = r0 + j, k = k0 + 2 * threadIdx.x;
         if (r < rows && k < Kp)        // Kp is even: the pair (k, k + 1) is inside the padded row
-            *reinterpret_cast<uint32_t*>(d + (size_t)r * Kp + k) = pack_bf16x2(tile[2 * threadIdx.x][j], tile[2 * threadIdx.x + 1][j]);
+            *reinterpret_cast<uint32_t*>(d + (size_t)r * Kp + k) = pack2(tile[2 * threadIdx.x][j], tile[2 * threadIdx.x + 1][j]);
     }
 }
 
@@ -374,7 +291,7 @@ __global__ void pack_im2col_kcontig_kernel(__nv_bfloat16* __restrict__ dst, cons
                 v[j] = (kk0 + j < NB * L && ls >= 0 && ls < L) ? xrow[(size_t)q * G * Cin * L + ls] : 0.f;
                 if (++l == L) { l = 0; ++q; }
             }
-            *reinterpret_cast<uint4*>(drow + kk0) = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+            *reinterpret_cast<uint4*>(drow + kk0) = make_uint4(pack2(v[0], v[1]), pack2(v[2], v[3]), pack2(v[4], v[5]), pack2(v[6], v[7]));
         }
     }
 }
